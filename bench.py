@@ -4,6 +4,10 @@ measured on the path `north_star` shards: the tile-parallel sliding-window evalu
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torch.distributed.run)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR
+
+--dump-outputs DIR: after the K timed rounds the blend rank writes what the last timed round computed as DIR/<name>.npy
+(see `dump_outputs`), so that two builds of the project can be compared output for output on identical seeded inputs.
 
 Workload.  A synthetic clip in the geometry of BASELINE.json configs[4] (480 x 853 frames -> two 480 x 720 spatial
 tiles per 41-frame temporal window, stride 8; reference evaluation/video_depth/launch_aether.py:81-287) is evaluated by
@@ -50,6 +54,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree: no __pycache__ there
 
 LATENT_FRAMES, LAT_H, LAT_W = 11, 60, 90
 TEXT_LEN, TEXT_DIM = 226, 4096
@@ -241,6 +246,33 @@ class SyntheticClip:
         return self._cache[key]
 
 
+DUMP_SAMPLE = 1 << 21          # elements kept of a larger output: the four outputs stay well under 64 MB together
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """Write every array of `arrays` (name -> numpy array or torch tensor) as <out_dir>/<name>.npy: float64 stays float64,
+    everything else becomes float32.  An array of more than DUMP_SAMPLE elements is replaced by the DUMP_SAMPLE elements
+    of its flattened form at a fixed seeded set of indices (ascending order, seed 0: the same positions in every run and
+    every build)."""
+    import numpy as np
+    import torch
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        if isinstance(a, np.ndarray):
+            a = a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False)
+        else:
+            a = a.detach().to(a.dtype if a.dtype == torch.float64 else torch.float32).cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        total += a.nbytes
+        if total > DUMP_MAX_BYTES:
+            raise ValueError(f"--dump-outputs: more than {DUMP_MAX_BYTES} bytes of outputs")
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def gpu_library_forward_ms(dev, reps: int = 3):
     """One DiT forward at the bench shape through stock PyTorch (oracle modules in bf16 on the GPU)."""
     import torch
@@ -338,10 +370,16 @@ def run_product(args):
     rounds = warmup + args.steps + n_e2e
     clip = SyntheticClip(clip_frames_for_tiles(rounds * world), CLIP_H, CLIP_W, dev)
     stats = {}
+    last_tile = []          # --dump-outputs: what the pipeline call of this rank's latest tile returned
+
+    def tile_pipe(*a, **kw):
+        last_tile[:] = [pipe(*a, **kw)]
+        return last_tile[0]
+
     # the evaluation decodes rgb for every tile like the reference (skip_unused_rgb=False): a round is a complete
     # configs[1] generation, nothing of it is skipped
-    run = TileParallelRun(pipe, clip, tile_steps, clip.shape[1], seed=3407, rank=rank, world_size=world, device=dev,
-                          skip_unused_rgb=False, stats=stats)
+    run = TileParallelRun(tile_pipe if args.dump_outputs else pipe, clip, tile_steps, clip.shape[1], seed=3407,
+                          rank=rank, world_size=world, device=dev, skip_unused_rgb=False, stats=stats)
     assert run.n_rounds == rounds, (run.n_rounds, rounds)
 
     def barrier():
@@ -384,6 +422,13 @@ def run_product(args):
     timed_stats = dict(stats)
     run.finish_stats_reset()
     value = world * LATENT_FRAMES * args.steps * (tile_steps / DENOISE_STEPS) / (elapsed_ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        # the last timed round: the pipeline outputs of its tile on this rank, and the blended disparity frames that
+        # no later window changes any more (what fetch_finalized hands a caller; the e2e rounds push more windows)
+        rgb, disp, ray = last_tile[0]
+        upto = run.plan.tiles[run.blend.windows_done * run.plan.n_spatial].t_start
+        dump_outputs(args.dump_outputs, {"tile_rgb": rgb, "tile_disparity": disp, "tile_raymap": ray,
+                                         "blended_disparity": run.blend.final[:upto]})
 
     # ---- e2e: the same round with host buffers (host uint8 frames in pinned memory in, finalised blended frames out)
     clip.host_mode = True
@@ -519,7 +564,13 @@ def main():
     ap.add_argument("--no-gpu-library-baseline", action="store_true")
     ap.add_argument("--no-strong-leg", action="store_true", help="skip the fixed-clip 4-step strong-scaling leg")
     ap.add_argument("--no-exchange-check", action="store_true", help="skip the golden check of the exchange + blend")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed round as DIR/<name>.npy (float32/float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1 (the number of timed rounds)")
+    if args.dump_outputs and args.impl != "product":
+        ap.error("--dump-outputs needs --impl product (the reference arm computes no outputs)")
     if args.impl == "reference":
         run_reference(args)
     else:

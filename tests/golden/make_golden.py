@@ -115,11 +115,21 @@ def make_sliding():
 
             def manual_seed(self, s):
                 return self
+        # the scale of every blend link, in call order (spatial links window by window, then the temporal chain):
+        # compute_scale sums fp32 products with torch.sum, whose order follows the host's thread count
+        scales, ref_scale = [], EVD.compute_scale
+
+        def recording_scale(*a, **k):
+            s = ref_scale(*a, **k)
+            scales.append(float(s))
+            return s
         torch.Generator = _Gen
+        EVD.compute_scale = recording_scale
         try:
             rgb, disp = EVD.process_with_sliding_window(fp, obs, num_inference_step=4, total_frames=t, seed=3407)
         finally:
             torch.Generator = orig
+            EVD.compute_scale = ref_scale
         assert len(fp.calls) == len(plan.tiles)
         tiles = np.array([[tl.t_start, tl.t_end, tl.h_start, tl.h_end, tl.w_start, tl.w_end] for tl in plan.tiles],
                          dtype=np.int64)
@@ -129,13 +139,17 @@ def make_sliding():
                             disparity_abs_sum=np.float64(np.abs(disp).sum()),
                             rgb_sub=subsample(rgb, (8, 32, 32, 1)), rgb_shape=np.array(rgb.shape))
         print(f"sliding_{name}.npz", disp.shape, disp.dtype, len(plan.tiles), "tiles")
+        all_scales[name] = np.array(scales, dtype=np.float64)
 
+    all_scales = {}
     run(57, 480, 720, "temporal")        # 3 temporal windows, no spatial tiling (windows stay fp32)
     run(49, 480, 853, "horizontal")      # 2 temporal x 2 horizontal tiles (overlap 587 px, SURVEY.md 8d config 5)
     run(41, 600, 720, "vertical")        # 1 temporal x 2 vertical tiles
     run(129, 480, 853, "long")           # 12 temporal x 2 horizontal = 24 tiles: the chain of BASELINE configs[4]
     #                                      (512 frames -> 60 x 2 tiles) at a quarter of its length, incl. the
     #                                      irregular last window at t - 41
+    np.savez_compressed(HERE / "sliding_scales.npz", **all_scales)
+    print("sliding_scales.npz", {k: len(v) for k, v in all_scales.items()})
 
 
 def make_pipeline():

@@ -117,6 +117,30 @@ def test_committed_multi_gpu_line_and_launch_shares_are_consistent(tmp_path):
     assert out.read_text() == (ROOT / "profiles" / "r2_bench_launch_shares.md").read_text()
 
 
+def test_bench_dump_outputs_and_argument_checks(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 stays float64, anything else is written as float32, a large output is reduced to
+    the same seeded positions in every run, and the dump never exceeds 64 MB.  --steps below 1 is refused."""
+    import subprocess
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)      # bench.py sets it at import
+    import bench
+    n = bench.DUMP_SAMPLE
+    big = np.arange(n + 12345, dtype=np.float32)                                    # value = position
+    bench.dump_outputs(tmp_path / "a", {"big": big, "small": torch.arange(6, dtype=torch.bfloat16).reshape(2, 3),
+                                        "f64": np.linspace(0.0, 1.0, 7)})
+    bench.dump_outputs(tmp_path / "b", {"big": 2 * big})
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and a.shape == (n,) and np.all(np.diff(a) > 0)
+    assert np.array_equal(b, 2 * a)
+    small = np.load(tmp_path / "a" / "small.npy")
+    assert small.dtype == np.float32 and np.array_equal(small, np.arange(6.0).reshape(2, 3))
+    assert np.load(tmp_path / "a" / "f64.npy").dtype == np.float64
+    with pytest.raises(ValueError):
+        bench.dump_outputs(tmp_path / "c", {f"x{i}": np.zeros(n, np.float64) for i in range(5)})
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "d")]):
+        r = subprocess.run([sys.executable, str(ROOT / "bench.py"), *bad], capture_output=True, text=True)
+        assert r.returncode == 2 and "error" in r.stderr, (bad, r.stderr)
+
+
 def test_library_has_no_libcuda_dependency():
     """The .so must load on a machine without the CUDA driver (driver entry points are resolved at run time)."""
     import subprocess
@@ -243,8 +267,11 @@ def _pose_worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_rel_pose_windows_gloo_world2():
+def test_rel_pose_windows_gloo_world2(monkeypatch):
     import torch.multiprocessing as mp
+    # the windows live on the GPU when one is visible, and gloo's send / recv carry host tensors only: the workers see
+    # no GPU, as on a machine without one
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
